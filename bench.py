@@ -130,8 +130,8 @@ _REF = {}
 
 
 def reference_kind():
-    """"reference" when the unmodified dynesty is importable on this box (the git-ignored offline
-    install baseline/_ref, or /root/reference in the build container), else "port" (the oracle)."""
+    """"reference" when the unmodified dynesty is importable (a dynesty checkout or its git-ignored copy
+    oracle/_ref, oracle/refshim.py), else "port" (the oracle)."""
     from oracle import refshim
     return 'reference' if refshim.available() else 'port'
 
@@ -229,7 +229,7 @@ def run_reference(args, cfg):
     if pool is not None:
         pool.close()
     val = tot_p / tot_t
-    who = ("dynesty RWalkSampler.sample (unmodified reference, baseline/_ref)" if kind == 'reference'
+    who = ("dynesty RWalkSampler.sample (unmodified reference)" if kind == 'reference'
            else "oracle rwalk")
     sample = "%d %s chains x %d walks per step on %d processes" % (nchains, who, cfg['walks'], cores)
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": "proposals/s", "n_gpus": args.gpus,
@@ -285,6 +285,23 @@ class ClockSampler:
 
 
 # ----------------------------------------------------------------------------- GPU arm
+RWALK_OUTPUTS = ('u', 'v', 'logl', 'n_accept', 'n_reject', 'ncall')
+
+
+def dump_outputs(outdir, ctx, d_out, Q, n, fused_world):
+    """--dump-outputs: what the last timed step returned to its caller -- rank 0's queue of Q chains (end point u,
+    its prior transform v and logl, and the chain counters) -- as DIR/<name>.npy in float64 (the counters exactly).
+    With the fused exchange the step writes into the peer window, so the rows are read from there."""
+    if fused_world:
+        o = ctx.peer_gathered(fused_world * Q, n, RWALK_OUTPUTS[3:])
+        o = {k: v[:Q] for k, v in o.items()}
+    else:
+        o = {k: d_out[k].cpu().numpy() for k in RWALK_OUTPUTS}
+    os.makedirs(outdir, exist_ok=True)
+    for k in RWALK_OUTPUTS:
+        np.save(os.path.join(outdir, k + '.npy'), np.ascontiguousarray(o[k], dtype=np.float64))
+
+
 def e2e_plugin(args, cfg, ctx, model, u_live, loglstar, scale, Q, walks):
     """The plug-in path a dynesty user drives, timed per queue fill on HOST data (every H2D / D2H inside):
       prepare_sampler : B200RWalkSampler.prepare_sampler(points=<list of Q rows>, axes=<Q axes handles>, seeds) +
@@ -292,11 +309,11 @@ def e2e_plugin(args, cfg, ctx, model, u_live, loglstar, scale, Q, walks):
       dynesty_fill_queue : the UNMODIFIED reference's own Sampler._fill_queue (sampler.py:676-717) with
                         bound=B200MultiEllipsoid, sample=B200RWalkSampler, pool=B200Pool, queue_size=Q -- Q x
                         propose_live (start row, get_random_axes, bound.contains) + prepare_sampler + map; only
-                        when the reference install (baseline/_ref) is present on this box."""
+                        when the reference is importable (oracle/refshim.py)."""
     import importlib
     from dynesty_b200 import _lib, samplers as S, bounding as B
     from dynesty_b200.pool import B200Pool
-    n, steps = cfg['ndim'], max(3, args.steps)
+    n, steps = cfg['ndim'], args.steps
     ctx.set_pointer_mode(_lib.PTR_HOST)
     out = {"unit": "proposals/s", "queue_size": Q, "walks": walks}
     rng = np.random.default_rng(SEED)
@@ -370,7 +387,7 @@ def e2e_plugin(args, cfg, ctx, model, u_live, loglstar, scale, Q, walks):
     out["dynesty_fill_queue"] = {"value": Q * walks * steps / dt, "ms_per_fill": 1e3 * dt / steps,
                                  "ms_per_fill_inside_the_plugin": 1e3 * mine[0] / steps,
                                  "ms_per_fill_dynesty_python": 1e3 * (dt - mine[0]) / steps,
-                                 "sampler": "unmodified dynesty.NestedSampler (baseline/_ref) with the B200 bound / sampler / pool",
+                                 "sampler": "unmodified dynesty.NestedSampler with the B200 bound / sampler / pool",
                                  "note": "dynesty's own per-slot Python (rstate.choice, get_random_axes, contains, SeedSequence.spawn) "
                                          "is the part outside the plug-in; it is why dynesty_b200.nested proposes a whole queue at once"}
     return out
@@ -550,6 +567,9 @@ def run_b200(args, cfg):
         dist.barrier()
     # clock ramp: ~0.7 s of the same kernel before timing, so that the nvidia-smi sampler has
     # samples under load.  N>1: a FIXED step count (every rank must issue the same exchanges).
+    # The timed steps start from the proposal RNG and chain counter as they are here, so that
+    # their inputs do not depend on how many ramp steps fit into the time.
+    rng_state, chain_next = rng.bit_generator.state, state['chain']
     if world > 1:
         for _ in range(2500):
             step_dev()
@@ -558,6 +578,7 @@ def run_b200(args, cfg):
         while time.perf_counter() < t_ramp:
             step_dev()
     torch.cuda.synchronize()
+    rng.bit_generator.state, state['chain'] = rng_state, chain_next
 
     def barrier():
         if world > 1:
@@ -579,6 +600,8 @@ def run_b200(args, cfg):
         kern_ms.append(ctx.last_kernel_ms())
     barrier()
     dev_ms = sum(a.elapsed_time(b) for a, b in ev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx, d_out, Q, n, world if fused else 0)
     # ---- timed: end to end through the plug-in call with host buffers
     barrier()
     t0 = time.perf_counter()
@@ -805,6 +828,8 @@ def main():
     ap.add_argument('--ramp', type=float, default=0.7, help='seconds of untimed steps before timing (clock ramp; 0 under ncu)')
     ap.add_argument('--exchange', default='fused', choices=['fused', 'nccl'],
                     help='N>1: how the finished chains reach every rank')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed device step as DIR/<name>.npy (float64)')
     args = ap.parse_args()
     cfg = WORKLOADS[args.workload]
     if args.impl == 'reference':

@@ -1,8 +1,9 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference.
 
-TEST INFRASTRUCTURE.  Run in the build container (needs /root/reference):
+TEST INFRASTRUCTURE.  Needs the reference: a dynesty checkout or its copy oracle/_ref
+(oracle/refshim.py):
 
-    python -m oracle.make_golden
+    python -m oracle.make_golden [bounding friends chains dynamic]    (default: all)
 
 Every output array below is produced by the reference's own functions
 (dynesty 3.0.0+ @ 99451618, imported through oracle/refshim.py); stochastic
@@ -371,18 +372,59 @@ def gen_friends(B):
     return out
 
 
-def main():
+def gen_dynamic():
+    """dynamic.npz: the reference's own dynamicsampler.weight_function / compute_weights and
+    utils.compute_integrals evaluated on the results of one device-loop run (3-D Gaussian, nlive 100, multi /
+    rwalk, rounds of 10) made on the oracle backend (tests/fake_backend.py).  The inputs are stored with the
+    outputs, so tests/test_dynamic.py and tests/test_oracle_nsloop.py compare with the reference without it."""
+    import sys
+    import types
+    import pytest
+    sys.path.insert(0, os.path.dirname(OUT))          # tests/: the oracle backend
+    import fake_backend
+    from dynesty import dynamicsampler as RD, utils as RU
+    from dynesty_b200 import nested, likelihoods as DL
+    mp = pytest.MonkeyPatch()
+    try:
+        fake_backend.install(mp)
+        s = nested.NestedSampler(DL.gauss_test3d(), nlive=100, bound='multi', sample='rwalk', walks=8, seed=2)
+        res = s.run_nested(dlogz=0.1, loop='device', batch=10)
+    finally:
+        mp.undo()
+    out = {k: np.asarray(getattr(res, k)) for k in ('logl', 'logz', 'logvol', 'logwt', 'samples_n')}
+    R = types.SimpleNamespace(**out)
+    out['weight_bounds'] = np.array([RD.weight_function(R, a) for a in WEIGHT_ARGS], dtype=float)
+    out['zweight'], out['pweight'] = RD.compute_weights(R)
+    out['integrals_logwt'], out['integrals_logz'] = RU.compute_integrals(logl=out['logl'], logvol=out['logvol'])[:2]
+    np.savez_compressed(os.path.join(OUT, 'dynamic.npz'), **out)
+    return out
+
+
+# the weight_function arguments of dynamic.npz's 'weight_bounds', row by row (None = the defaults)
+WEIGHT_ARGS = (None, dict(pfrac=0.0), dict(pfrac=1.0, maxfrac=0.5, pad=3))
+
+
+FIXTURES = ('bounding', 'friends', 'chains', 'dynamic')
+
+
+def main(which=FIXTURES):
     os.makedirs(OUT, exist_ok=True)
     refshim.import_reference()
     from dynesty import bounding as B, internal_samplers as IS
-    gen_bounding(B)
-    gen_friends(B)
-    out = gen_chains(B, IS)
+    if 'bounding' in which:
+        gen_bounding(B)
+    if 'friends' in which:
+        gen_friends(B)
+    if 'chains' in which:
+        out = gen_chains(B, IS)
+        ku = [k for k in out if k.endswith('_logvols') and k.startswith('unif')]
+        print({k: len(out[k]) for k in ku})
+    if 'dynamic' in which:
+        gen_dynamic()
     print('wrote', OUT, {k: os.path.getsize(os.path.join(OUT, k))
                          for k in sorted(os.listdir(OUT))})
-    ku = [k for k in out if k.endswith('_logvols') and k.startswith('unif')]
-    print({k: len(out[k]) for k in ku})
 
 
 if __name__ == '__main__':
-    main()
+    import sys
+    main(sys.argv[1:] or FIXTURES)

@@ -21,19 +21,21 @@ def _free_port():
     return p
 
 
-def _run(rank, world, port, outdir, sample='rwalk'):
+def _run(rank, world, port, outdir, sample='rwalk', patch=None):
+    """One rank of the run.  `patch`: the calling test's monkeypatch when the rank runs inside the pytest process,
+    so that the stand-in backend and the environment are restored when the test ends (later tests in the same
+    session, the GPU ones included, must see the real library)."""
     sys.path.insert(0, ROOT)
     sys.path.insert(0, os.path.join(ROOT, 'tests'))
-    os.environ.update(MASTER_ADDR='127.0.0.1', MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
+    patch = patch or pytest.MonkeyPatch()
+    for k, v in dict(MASTER_ADDR='127.0.0.1', MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world)).items():
+        patch.setenv(k, v)
     import torch.distributed as dist
     import fake_backend
     from dynesty_b200 import ops, likelihoods as DL, nested
     from dynesty_b200.dist import Comm
 
-    class MP:                       # minimal monkeypatch object
-        def setattr(self, obj, name, val):
-            setattr(obj, name, val)
-    fake_backend.install(MP())
+    fake_backend.install(patch)
     comm = None
     if world > 1:
         dist.init_process_group('gloo', rank=rank, world_size=world)
@@ -49,10 +51,10 @@ def _run(rank, world, port, outdir, sample='rwalk'):
 
 
 @pytest.mark.parametrize('sample', ['rwalk', 'rslice', 'unif'])
-def test_sharded_run_matches_single_rank(tmp_path, sample):
+def test_sharded_run_matches_single_rank(tmp_path, monkeypatch, sample):
     """rslice / unif fills return an unsigned `flags` array: the all-gather must carry it (ADVICE r1)."""
     import torch.multiprocessing as mp
-    _run(0, 1, 0, str(tmp_path), sample)
+    _run(0, 1, 0, str(tmp_path), sample, monkeypatch)
     port = _free_port()
     mp.spawn(_run, args=(2, port, str(tmp_path), sample), nprocs=2, join=True)
     a = np.load(tmp_path / ('%s_r0_w1.npz' % sample))

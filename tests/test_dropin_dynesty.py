@@ -2,18 +2,18 @@
 ``dynesty.NestedSampler`` through its official seams (bound= / sample= / pool=), the same
 way the reference's tests/test_bound_interface.py and tests/test_sampler_interface.py
 plug in user classes.  Numerics come from the oracle-backed stand-in (tests/fake_backend.py);
-what is pinned is the interface contract.  Skipped where the reference is absent (GPU box).
+what is pinned is the interface contract.  The tests that run the reference skip where neither a dynesty
+checkout nor its copy oracle/_ref is present (oracle/refshim.py).
 """
 import numpy as np
 import pytest
 
 from oracle import refshim
 
-pytestmark = pytest.mark.skipif(not refshim.available(), reason="reference not present")
-
-
 @pytest.fixture(scope='module')
 def dynesty():
+    if not refshim.available():
+        pytest.skip("reference not present")
     return refshim.import_reference()
 
 
@@ -73,7 +73,7 @@ def test_reference_bound_with_b200_sampler(dynesty, fake_ops):
     assert abs(ns.results['logz'][-1] - 3 * (-np.log(20.))) < 5 * ns.results['logzerr'][-1] + 0.1
 
 
-def test_sampler_requires_model(dynesty):
+def test_sampler_requires_model():
     c, b, s = _classes()
     with pytest.raises(ValueError):
         s.B200RWalkSampler(walks=5)

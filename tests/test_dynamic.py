@@ -1,12 +1,14 @@
 """CPU tier: dynesty_b200/dynamic.py -- the dynamic sampler whose baseline and batches are device rounds.  The merge is
 checked against a literal restatement of the reference's ``combine_runs`` loop (dynamicsampler.py:1500-1560), the
-weight function against the reference's own ``weight_function`` when the reference is importable, and a whole run
+weight function against stored outputs of the reference's own ``weight_function``, and a whole run
 against the analytic evidence on the oracle backend."""
+import os
+
 import numpy as np
 import pytest
 
 from dynesty_b200 import dynamic as D, likelihoods as DL
-from oracle import refshim
+from oracle import make_golden
 
 
 def _loop_merge(ls, ns, ln, nn, logl_min):
@@ -43,22 +45,15 @@ def test_merge_two_equals_the_reference_loop(seed):
     assert np.all(np.diff(m['logl']) >= 0)
 
 
-@pytest.mark.skipif(not refshim.available(), reason="reference not present")
-def test_weight_function_matches_reference(fake_ops):
-    refshim.import_reference()
-    from dynesty import dynamicsampler as RD
-    from dynesty_b200 import nested
-    m = DL.gauss_test3d()
-    s = nested.NestedSampler(m, nlive=100, bound='multi', sample='rwalk', walks=8, seed=2)
-    res = s.run_nested(dlogz=0.1, loop='device', batch=10)
-
-    class R:           # what the reference's weight functions read off a Results object
-        logl, logz, logvol, logwt, samples_n = res.logl, res.logz, res.logvol, res.logwt, res.samples_n
-    for args in (None, dict(pfrac=0.0), dict(pfrac=1.0, maxfrac=0.5, pad=3)):
-        a = RD.weight_function(R, args)
+def test_weight_function_matches_reference():
+    """The reference's own weight_function / compute_weights on the results of a device-loop run (oracle backend),
+    stored with those results in tests/golden/dynamic.npz by oracle/make_golden.py."""
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'dynamic.npz'))
+    res = {k: g[k] for k in ('logl', 'logz', 'logvol', 'logwt', 'samples_n')}
+    for args, a in zip(make_golden.WEIGHT_ARGS, g['weight_bounds']):
         b = D.weight_function(res, args)
         assert a[0] == b[0] and a[1] == b[1]
-    za, pa = RD.compute_weights(R)
+    za, pa = g['zweight'], g['pweight']
     zb, pb = D.compute_weights(res)
     np.testing.assert_allclose(za, zb, rtol=1e-9)
     np.testing.assert_allclose(pa, pb, rtol=1e-12)

@@ -5,8 +5,8 @@ drop-in claim of SURVEY.md 8(b), end to end: the reference's own ``Sampler`` cal
 ``sample.prepare_sampler / sample / tune`` (sampler.py:469-510, 676-778) and every one of
 those lands in libb200nest.so.
 
-The reference travels to the GPU box only as the git-ignored offline install
-``baseline/_ref`` (oracle/refshim.py); the tests skip when it is absent.  The same seams
+The reference is a dynesty checkout or the git-ignored copy ``oracle/_ref`` that build() makes of
+one (oracle/refshim.py); the tests skip when neither is present.  The same seams
 are exercised on CPU with the oracle-backed stand-in in tests/test_dropin_dynesty.py.
 """
 import math
@@ -17,7 +17,7 @@ import pytest
 from oracle import refshim
 
 pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not refshim.available(), reason="reference install (baseline/_ref) not present")]
+              pytest.mark.skipif(not refshim.available(), reason="reference (oracle/refshim.py) not present")]
 
 KW = dict(use_pool={'prior_transform': False, 'loglikelihood': False})
 
