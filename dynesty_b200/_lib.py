@@ -113,6 +113,9 @@ SYMBOLS = {
     'b2n_ns_bound_updated': (C.c_int, [_P]),
     'b2n_ns_update_bound': (C.c_int, [_P, _I, _D, _P, _P, _P]),
     'b2n_ns_get_bound': (C.c_int, [_P, _I, _P, _P, _P, _P, _P, _P]),
+    'b2n_ns_update_friends': (C.c_int, [_P, _I, _D, _I, _I, _P, _P, _P]),
+    'b2n_ns_set_friends': (C.c_int, [_P, _I, _P, _P, _P, _P, _D]),
+    'b2n_ns_get_friends': (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P]),
     'b2n_ns_reserve_dead': (C.c_int, [_P, _L]),
     'b2n_ns_get_live': (C.c_int, [_P, _P, _P, _P]),
     'b2n_ns_get_dead': (C.c_int, [_P, _L, _L, _P, _P, _P, _P, _P]),

@@ -102,6 +102,7 @@ struct b2n_ctx {
     // resident bound
     int bK = 0, bn = 0;
     DevBuf b_ctrs, b_ams, b_axesT, b_logvols;
+    unsigned long long bound_serial = 0;   // bumped by every b2n_bound_set / b2n_bound_set_dev (who holds the bound)
     std::vector<double> h_logvols;
     // staging (host-pointer mode) and scratch
     DevBuf in0, in1, in2, in3, out0, out1, out2, out3, out4, out5, out6, out7;
@@ -136,6 +137,14 @@ void b2n_ns_release(b2n_ctx* ctx);
 void b2n_friends_release(b2n_ctx* ctx);
 int b2n_bound_set_dev(b2n_ctx* ctx, int K, int nc, const double* dctrs, const double* dams, const double* daxes,
                       const double* h_logvols);
+// friends mode of the device-resident rounds (b2n_friends.cu, used by b2n_ns.cu; all pointers device arrays):
+//   y = x @ T for N rows (friends_transform_kernel); cov *= f^2, am /= f^2, axes *= f, axes_inv /= f (the host class's
+//   scale_to_logvol arithmetic); UniformBoundSampler.sample with the centres `ctrs` (N rows), device-paced (ctx->dyn)
+int b2n_friends_transform_dev(b2n_ctx* ctx, const double* x, int N, int n, const double* T, double* y);
+int b2n_friends_rescale_dev(b2n_ctx* ctx, int n, double* cov, double* am, double* axes, double* axes_inv, double f);
+int b2n_friends_unif_dev(b2n_ctx* ctx, const b2n_chain_args* a, int N, int kind, const double* ctrs, const double* ctrs_t,
+                         const double* axes, const double* axes_inv, double* u, double* v, double* logl, int32_t* ncall,
+                         int32_t* nprop, uint32_t* flags);
 
 // gather-mode plumbing shared by the chain entry points (b2n_peer.cu).  b2n_peer_begin: when
 // gather mode is on, point the 7 output arrays at this rank's rows of its own window and fill

@@ -263,6 +263,7 @@ int b2n_bound_set(b2n_ctx* ctx, int32_t K, int32_t nc, const double* ctrs, const
     }
     ctx->bK = K;
     ctx->bn = nc;
+    ctx->bound_serial++;
     return B2N_OK;
 }
 
@@ -296,6 +297,7 @@ int b2n_bound_set_dev(b2n_ctx* ctx, int K, int nc, const double* dctrs, const do
     B2N_CUDA(ctx, cudaMemcpyAsync(ctx->b_logvols.p, ctx->h_logvols.data(), (size_t)K * sizeof(double), cudaMemcpyHostToDevice, st));
     ctx->bK = K;
     ctx->bn = nc;
+    ctx->bound_serial++;
     return B2N_OK;
 }
 

@@ -228,6 +228,19 @@ __global__ void friends_scale_kernel(double* __restrict__ m, size_t count, doubl
     for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < count; e += (size_t)gridDim.x * blockDim.x) m[e] *= f;
 }
 
+// _B200Friends.scale_to_logvol (bounding.py:765-774 / 1031-1040) element by element: cov * f**2, am / f**2, axes * f,
+// axes_inv / f -- the same IEEE operations as the numpy expressions (a division stays a division), so that the enlarged
+// bound of the device rounds equals the host route's bit for bit
+__global__ void friends_rescale_kernel(double* __restrict__ cov, double* __restrict__ am, double* __restrict__ axes,
+                                       double* __restrict__ axes_inv, size_t count, double f, double f2) {
+    for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < count; e += (size_t)gridDim.x * blockDim.x) {
+        cov[e] *= f2;
+        am[e] /= f2;
+        axes[e] *= f;
+        axes_inv[e] /= f;
+    }
+}
+
 // distance of the transformed query xt to centre row ct (kind 0: squared Euclidean, 1: Chebyshev)
 __device__ __forceinline__ double friends_dist(const double* __restrict__ ct, const double* xt, int n, int kind) {
     double s = 0.0;
@@ -275,12 +288,19 @@ struct FriendsUnifParams {
     double *u, *v, *logl;
     int *ncall, *nprop;
     uint32_t* flags;
+    const B2nDyn* dyn;     // device-paced launch (friends mode of b2n_ns.cu): threshold / chain ids in HBM
 };
 
 template <int LIKE>
 __global__ void __launch_bounds__(128) friends_unif_kernel(const FriendsUnifParams p) {
     extern __shared__ double fsm[];
     const int n = p.n, N = p.N;
+    double loglstar_ = p.loglstar;
+    uint64_t chain0_ = p.chain0;
+    if (p.dyn) {
+        if (p.dyn->skip) return;
+        loglstar_ = p.dyn->loglstar; chain0_ = p.dyn->chain0;
+    }
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, wpb = blockDim.x >> 5;
     double* uu = fsm + (size_t)warp * 5 * n;
     double* z = uu + n;
@@ -290,7 +310,7 @@ __global__ void __launch_bounds__(128) friends_unif_kernel(const FriendsUnifPara
     const double inv_n = 1.0 / (double)n;
     for (int64_t q = (int64_t)blockIdx.x * wpb + warp; q < p.Q; q += (int64_t)gridDim.x * wpb) {
         ChainRng g;
-        g.init(p.seed, p.chain0 + (uint64_t)q);
+        g.init(p.seed, chain0_ + (uint64_t)q);
         int ncall = 0, nprop = 0;
         uint32_t fl = 0;
         double lcur = 0.0;
@@ -355,7 +375,7 @@ __global__ void __launch_bounds__(128) friends_unif_kernel(const FriendsUnifPara
             __syncwarp();
             lcur = warp_loglike<LIKE>(p.m, p.m.lmat, vv, work, lane);
             ncall++;
-            if (lcur > p.loglstar) done = true;
+            if (lcur > loglstar_) done = true;
         }
         __syncwarp();
         for (int i = lane; i < n; i += 32) { p.u[q * n + i] = uu[i]; p.v[q * n + i] = vv[i]; }
@@ -618,6 +638,7 @@ int b2n_friends_unif_batch(b2n_ctx* ctx, const b2n_chain_args* a, double* u, dou
     p.m = m; p.n = n; p.N = f->N; p.kind = f->kind; p.draw_only = draw_only;
     p.ctrs = f->ctrs.as<double>(); p.ctrs_t = f->ctrs_t.as<double>(); p.axes = f->axes.as<double>(); p.axes_inv = f->axes_inv.as<double>();
     p.dimflags = (const uint32_t*)dfl_in; p.loglstar = a->loglstar; p.seed = a->seed; p.chain0 = a->chain0; p.Q = Q;
+    p.dyn = nullptr;
     void *du, *dv, *dl, *dnc, *dnp, *dfl;
     B2N_TRY(b2n_out(ctx, ctx->out0, u, (size_t)Q * n * sizeof(double), &du));
     B2N_TRY(b2n_out(ctx, ctx->out1, v, (size_t)Q * n * sizeof(double), &dv));
@@ -647,3 +668,60 @@ int b2n_friends_unif_batch(b2n_ctx* ctx, const b2n_chain_args* a, double* u, dou
 }
 
 }  // extern "C"
+
+// ---- friends mode of the device-resident rounds (b2n_ns.cu) -------------------------------------------------------
+int b2n_friends_transform_dev(b2n_ctx* ctx, const double* x, int N, int n, const double* T, double* y) {
+    friends_transform_kernel<<<(unsigned)(((size_t)N * 32 + 255) / 256), 256, 0, ctx->stream>>>(x, N, n, T, y);
+    B2N_LAUNCH_CHECK(ctx);
+    return B2N_OK;
+}
+
+int b2n_friends_rescale_dev(b2n_ctx* ctx, int n, double* cov, double* am, double* axes, double* axes_inv, double f) {
+    const size_t nn = (size_t)n * n;
+    friends_rescale_kernel<<<(unsigned)std::min<size_t>((nn + 255) / 256, 64), 256, 0, ctx->stream>>>(
+        cov, am, axes, axes_inv, nn, f, pow(f, 2.0));
+    B2N_LAUNCH_CHECK(ctx);
+    return B2N_OK;
+}
+
+// One device-paced launch of friends_unif_kernel for the K chains of a round: the centres are the run's live set as it
+// stands (the reference re-points bound.ctrs = live_u before every proposal, sampler.py:479-482), ctrs_t its rows
+// times axes_inv, kept current by the round's commit kernel.  Threshold and chain ids come from ctx->dyn.
+int b2n_friends_unif_dev(b2n_ctx* ctx, const b2n_chain_args* a, int N, int kind, const double* ctrs, const double* ctrs_t,
+                         const double* axes, const double* axes_inv, double* u, double* v, double* logl, int32_t* ncall,
+                         int32_t* nprop, uint32_t* flags) {
+    if (!ctx->dyn.active || ctx->ptr_mode != B2N_PTR_DEVICE) return b2n_fail(ctx, B2N_ERR_ARG, "b2n_friends_unif_dev: device-paced launches only");
+    ctx->dyn.cpc = 1;
+    if (ctx->dyn.plan_only) return B2N_OK;
+    if (a->model_id < 0 || a->model_id >= (int)ctx->models.size()) return B2N_ERR_ARG;
+    const B2nModel m = ctx->models[a->model_id];
+    const int n = a->ndim;
+    const int64_t Q = a->nchain;
+    if (n != m.ndim || a->ncdim != n || Q < 1 || N < 1) return B2N_ERR_ARG;
+    const void* dfl_in = nullptr;
+    std::vector<uint32_t> fl;
+    if (a->dimflags) {
+        fl.assign(a->dimflags, a->dimflags + n);
+        B2N_TRY(b2n_in_host(ctx, ctx->in3, fl.data(), fl.size() * sizeof(uint32_t), &dfl_in));
+    }
+    FriendsUnifParams p;
+    p.m = m; p.n = n; p.N = N; p.kind = kind; p.draw_only = 0;
+    p.ctrs = ctrs; p.ctrs_t = ctrs_t; p.axes = axes; p.axes_inv = axes_inv;
+    p.dimflags = (const uint32_t*)dfl_in; p.loglstar = a->loglstar; p.seed = a->seed; p.chain0 = a->chain0; p.Q = Q;
+    p.u = u; p.v = v; p.logl = logl; p.ncall = ncall; p.nprop = nprop; p.flags = flags;
+    p.dyn = ctx->dyn.dev;
+    const int threads = 128, wpb = threads / 32;
+    const size_t smem = (size_t)wpb * 5 * n * sizeof(double);
+    if (smem > (size_t)ctx->max_smem_optin) return b2n_fail(ctx, B2N_ERR_UNSUPPORTED, "ndim too large for the friends kernel");
+    const int64_t blocks = (Q + wpb - 1) / wpb;
+#define CALL(L)                                                                                                   \
+    if (smem > 48 * 1024)                                                                                         \
+        B2N_TRY(b2n_func_smem(ctx, (const void*)(friends_unif_kernel<L>), (size_t)(smem))); \
+    friends_unif_kernel<L><<<(unsigned)blocks, threads, smem, ctx->stream>>>(p);
+    B2N_TIME_BEGIN(ctx);
+    B2N_DISPATCH_LIKE(m.like_kind, CALL)
+    B2N_TIME_END(ctx);
+#undef CALL
+    B2N_LAUNCH_CHECK(ctx);
+    return B2N_OK;            // the commit kernel of the round folds the flags (draw limit: 0x80000000)
+}

@@ -35,6 +35,11 @@
 #include <math_constants.h>
 
 #define B2N_NS_DRIVER_CHAIN 0x4000000000000000ULL   // Philox chain id space of the round driver
+// Philox chain id space of the bootstrap realisations of the friends bounds' device updates (b2n_ns_update_friends):
+// realisation b of an update made at round r is the chain B2N_NS_FRIENDS_BOOT_CHAIN + (r << 8) + b, b < 256 --
+// disjoint from the live-point initialisation (2^61 + i), the round driver (2^62 + r) and the chains (chain0 + r K + c)
+#define B2N_NS_FRIENDS_BOOT_CHAIN 0x6000000000000000ULL
+#define B2N_NS_FRIENDS_MAX_BOOT 255
 #define B2N_NS_THREADS 1024
 
 struct NsScalars {
@@ -68,6 +73,11 @@ struct NsDev {
     int *o_i0, *o_i1, *o_ncall;
     uint32_t* o_flags;
     const double *ctrs, *ams, *logvols;      // resident bound
+    // friends mode (RadFriends / SupFriends, b2n_ns_update_friends / b2n_ns_set_friends): one ball / cube of common
+    // shape around every live point.  Kell = 1 and no contains test (a start point is a live point, hence a centre).
+    int friends, pad1;
+    const double* fr_axes_inv;   // uniform sampler only: the commit refreshes the replaced rows of fr_ctrs_t =
+    double* fr_ctrs_t;           // live_u @ axes_inv (the transformed centres friends_unif_kernel counts q with)
 };
 
 struct b2n_ns {
@@ -94,6 +104,13 @@ struct b2n_ns {
     double *bd_ctrs = nullptr, *bd_covs = nullptr, *bd_ams = nullptr, *bd_axes = nullptr, *bd_axlens = nullptr,
            *bd_logvols = nullptr, *bd_points = nullptr;
     std::vector<double> bd_hlogvols;
+    // friends mode: the run's RadFriends / SupFriends bound (n x n each), allocated by the first friends entry point.
+    // fr_ready: a bound exists (fit or adopted); fr_am is the am_prev of the next update.
+    bool friends = false, fr_ready = false;
+    int fr_kind = 0, fr_ncl = 0;
+    double fr_logvol = 0.0, fr_radius = 0.0;
+    double *fr_cov = nullptr, *fr_am = nullptr, *fr_axes = nullptr, *fr_axinv = nullptr, *fr_ctrs_t = nullptr;
+    unsigned long long fr_serial = 0;  // ctx->bound_serial right after this run made its axes the resident bound
 };
 
 __device__ __forceinline__ double dev_logaddexp(double a, double b) {
@@ -230,8 +247,10 @@ __device__ __forceinline__ void ns_propose_body(const NsDev& s) {
         ell[c] = e;
     }
     __syncthreads();
-    // ---- bound.contains(start[:nc]) (sampler.py:485-489): a start outside forces a bound update
-    for (int c = warp; c < K; c += (nth >> 5)) {
+    // ---- bound.contains(start[:nc]) (sampler.py:485-489): a start outside forces a bound update.  Not with the
+    //      friends bounds: the start is a live point, i.e. a centre of the bound (distance 0), so the forced update
+    //      of sampler.py:485-489 can never fire
+    for (int c = warp; c < K && !s.friends; c += (nth >> 5)) {
         const double* x = s.live_u + (size_t)start[c] * n;
         double* d = dvec + warp * nc;
         bool inside = false;
@@ -364,6 +383,16 @@ __device__ __forceinline__ void ns_commit_body(const NsDev& s) {
         s.dead_v[dst] = s.live_v[src];
         s.live_u[src] = s.o_u[e];
         s.live_v[src] = s.o_v[e];
+    }
+    if (s.fr_ctrs_t) {      // friends mode, uniform sampler: transformed centres of the K new rows, with the arithmetic
+                            // of friends_transform_kernel (k ascending, fma) -- equal to a full re-transform bit for bit
+        for (int e = tid; e < K * n; e += nth) {
+            const int j = e / n, i = e - j * n;
+            const double* x = s.o_u + (size_t)j * n;
+            double acc = 0.0;
+            for (int k = 0; k < n; k++) acc = fma(x[k], __ldg(s.fr_axes_inv + (size_t)k * n + i), acc);
+            s.fr_ctrs_t[(size_t)cidx[j] * n + i] = acc;
+        }
     }
     // ---- evidence: ln X_j = ln X_0 + ln((N-j)/(N+1)); trapezoid weight with dX_j = X_j / (N-j) * 1/2 ..
     double wmax = -CUDART_INF;
@@ -579,6 +608,9 @@ static int ns_chain_call(b2n_ctx* ctx, b2n_ns* ns, bool plan_only) {
     if (ns->phase == 0) {
         if (plan_only) { ctx->dyn.cpc = 1; st = B2N_OK; }
         else st = b2n_unitcube_batch(ctx, &a, d.o_u, d.o_v, d.o_logl, d.o_ncall, d.o_flags);
+    } else if (d.sampler == 3 && ns->friends) {
+        st = b2n_friends_unif_dev(ctx, &a, d.N, ns->fr_kind, d.live_u, ns->fr_ctrs_t, ns->fr_axes, ns->fr_axinv, d.o_u,
+                                  d.o_v, d.o_logl, d.o_ncall, d.o_i0, d.o_flags);
     } else if (d.sampler == 3) {
         if (plan_only) { ctx->dyn.cpc = 1; st = B2N_OK; }
         else st = b2n_unif_batch(ctx, &a, d.o_u, d.o_v, d.o_logl, d.o_ncall, d.o_i0, d.o_flags);
@@ -617,6 +649,48 @@ static size_t ns_commit_smem(const NsDev& d) {
     return (NA + (NA & 1)) * 8 + (size_t)d.Kpad * 8 + NA * 4 + (size_t)d.Kpad * 4 + 64;
 }
 static size_t ns_sort_smem(const NsDev& d) { return (size_t)d.Npad * 12 + 64; }
+
+// A bound update is a chain of ~45 small dependent kernels with a dozen host round trips; with other replicas' chain
+// CTAs filling every SM each of them used to wait its turn (68 updates cost 2.5 s per run at 48 replicas in flight
+// against 0.18 s alone).  It runs on the context's HIGH-PRIORITY stream: its CTAs are placed before the pending CTAs
+// of normal-priority grids.  The main stream is idle here (the rounds were synchronised).
+struct StreamSwap {
+    b2n_ctx* c; cudaStream_t keep; bool on;
+    explicit StreamSwap(b2n_ctx* ctx) : c(ctx), keep(ctx->stream), on(ctx->own_stream && ctx->stream_hi != nullptr) {
+        if (on) { cudaStreamSynchronize(keep); c->stream = c->stream_hi; }
+    }
+    ~StreamSwap() { if (on) { cudaStreamSynchronize(c->stream_hi); c->stream = keep; } }
+};
+
+// ---- friends mode --------------------------------------------------------------------------------------------------
+static int ns_friends_alloc(b2n_ctx* ctx, b2n_ns* ns) {
+    if (ns->fr_cov) return B2N_OK;            // (kept with the run's other allocations across runs of the same shape)
+    const size_t n = ns->d.n, nn = n * n;
+    B2N_TRY(ns_alloc(ctx, ns, (void**)&ns->fr_cov, nn * 8));
+    B2N_TRY(ns_alloc(ctx, ns, (void**)&ns->fr_am, nn * 8));
+    B2N_TRY(ns_alloc(ctx, ns, (void**)&ns->fr_axes, nn * 8));
+    B2N_TRY(ns_alloc(ctx, ns, (void**)&ns->fr_axinv, nn * 8));
+    B2N_TRY(ns_alloc(ctx, ns, (void**)&ns->fr_ctrs_t, (size_t)ns->d.N * n * 8));
+    return B2N_OK;
+}
+
+// the common axes as the one-"ellipsoid" resident bound the chain kernels read (get_random_axes returns self.axes,
+// bounding.py:995-997 / 1262-1264).  The friends bounds have no ellipsoid centre: row 0 of the live set fills that slot, which no
+// kernel of this mode reads (the uniform sampler of this mode draws around the live points themselves).
+static int ns_friends_resident(b2n_ctx* ctx, b2n_ns* ns) {
+    B2N_TRY(b2n_bound_set_dev(ctx, 1, ns->d.n, ns->d.live_u, ns->fr_am, ns->fr_axes, &ns->fr_logvol));
+    ns->fr_serial = ctx->bound_serial;
+    return B2N_OK;
+}
+
+// make the bound in fr_* the run's bound: resident axes, centres = the live set, ctrs_t = live_u @ axes_inv (all N rows)
+static int ns_friends_adopt(b2n_ctx* ctx, b2n_ns* ns) {
+    NsDev& d = ns->d;
+    B2N_TRY(ns_friends_resident(ctx, ns));
+    B2N_TRY(b2n_friends_transform_dev(ctx, d.live_u, d.N, d.n, ns->fr_axinv, ns->fr_ctrs_t));
+    ns->friends = ns->fr_ready = true;
+    return B2N_OK;
+}
 
 extern "C" {
 
@@ -657,6 +731,8 @@ int b2n_ns_create(b2n_ctx* ctx, const b2n_ns_config* c, int64_t dead_capacity) {
     d.logl_max = c->use_logl_max ? c->logl_max : (double)INFINITY;
     ns->phase = c->unit_cube_phase ? 0 : 1;
     ns->bK = 0;
+    ns->friends = ns->fr_ready = false;          // every run starts in ellipsoid mode
+    d.friends = 0; d.fr_axes_inv = nullptr; d.fr_ctrs_t = nullptr;
     const size_t N = d.N, K = d.K;
     if (!reuse) {
         B2N_TRY(ns_alloc(ctx, ns, (void**)&d.live_u, N * n * 8));
@@ -779,9 +855,17 @@ int b2n_ns_run(b2n_ctx* ctx, int32_t max_rounds, int32_t check_every, b2n_ns_sta
     NsDev& d = ns->d;
     B2N_CUDA(ctx, cudaSetDevice(ctx->device));
     if (ctx->peer.total > 0) return b2n_fail(ctx, B2N_ERR_UNSUPPORTED, "b2n_ns_run: gather mode must be off");
+    d.friends = 0; d.fr_axes_inv = nullptr; d.fr_ctrs_t = nullptr;
     if (ns->phase == 0) {            // unit-cube rounds: no bound yet
         d.Kell = 1;
         d.ctrs = d.ams = d.logvols = nullptr;
+    } else if (ns->friends) {        // one common shape: the chains read its axes as the one resident "ellipsoid"
+        if (!ns->fr_ready) return b2n_fail(ctx, B2N_ERR_ARG, "friends mode: no bound yet (b2n_ns_update_friends / b2n_ns_set_friends)");
+        if (ctx->bound_serial != ns->fr_serial) B2N_TRY(ns_friends_resident(ctx, ns));   // someone replaced it since
+        d.Kell = 1;
+        d.ctrs = d.ams = d.logvols = nullptr;
+        d.friends = 1;
+        if (d.sampler == 3) { d.fr_axes_inv = ns->fr_axinv; d.fr_ctrs_t = ns->fr_ctrs_t; }
     } else {
         if (ctx->bK < 1 || ctx->bn != d.nc) return b2n_fail(ctx, B2N_ERR_ARG, "resident bound missing or of wrong dimension (b2n_bound_set)");
         if (!ctx->b_ctrs.p || !ctx->b_ams.p || !ctx->b_logvols.p || ctx->h_logvols.empty())
@@ -889,17 +973,8 @@ int b2n_ns_update_bound(b2n_ctx* ctx, int32_t multi, double enlarge, int32_t* ne
     b2n_ns* ns = ctx->ns;
     NsDev& d = ns->d;
     B2N_CUDA(ctx, cudaSetDevice(ctx->device));
-    // The update is a chain of ~45 small dependent kernels with a dozen host round trips; with other replicas' chain
-    // CTAs filling every SM each of them used to wait its turn (68 updates cost 2.5 s per run at 48 replicas in
-    // flight against 0.18 s alone).  It runs on the context's HIGH-PRIORITY stream: its CTAs are placed before the
-    // pending CTAs of normal-priority grids.  The main stream is idle here (the rounds were synchronised).
-    struct StreamSwap {
-        b2n_ctx* c; cudaStream_t keep; bool on;
-        explicit StreamSwap(b2n_ctx* ctx) : c(ctx), keep(ctx->stream), on(ctx->own_stream && ctx->stream_hi != nullptr) {
-            if (on) { cudaStreamSynchronize(keep); c->stream = c->stream_hi; }
-        }
-        ~StreamSwap() { if (on) { cudaStreamSynchronize(c->stream_hi); c->stream = keep; } }
-    } swap_(ctx);
+    if (ns->friends) return b2n_fail(ctx, B2N_ERR_ARG, "b2n_ns_update_bound: this run holds a friends bound (b2n_ns_update_friends)");
+    StreamSwap swap_(ctx);
     const int n = d.n, nc = d.nc, N = d.N;
     const double* pts = d.live_u;
     if (nc != n) {                  // the bound lives in the first ncdim coordinates (sampler.py:497)
@@ -974,6 +1049,97 @@ int b2n_ns_get_bound(b2n_ctx* ctx, int32_t max_ells, double* ctrs, double* covs,
     if (axes) B2N_CUDA(ctx, b2n_copy_sync(ctx, axes, ns->bd_axes, K * nn * 8, cudaMemcpyDeviceToHost));
     if (axlens) B2N_CUDA(ctx, b2n_copy_sync(ctx, axlens, ns->bd_axlens, K * nc * 8, cudaMemcpyDeviceToHost));
     if (logvols) memcpy(logvols, ns->bd_hlogvols.data(), K * 8);
+    return B2N_OK;
+}
+
+int b2n_ns_update_friends(b2n_ctx* ctx, int32_t kind, double enlarge, int32_t nboot, int32_t use_clustering,
+                          double* logvol, double* radius, int32_t* nclusters) {
+    if (!ctx || !ctx->ns || !ctx->ns->active || (kind != 0 && kind != 1) || !(enlarge > 0.0) || nboot < 0) return B2N_ERR_ARG;
+    if (nboot > B2N_NS_FRIENDS_MAX_BOOT) return b2n_fail(ctx, B2N_ERR_ARG, "b2n_ns_update_friends: nboot <= 255 (bootstrap chain ids)");
+    b2n_ns* ns = ctx->ns;
+    NsDev& d = ns->d;
+    if (d.nc != d.n) return b2n_fail(ctx, B2N_ERR_ARG, "the friends bounds need ncdim == ndim");
+    B2N_CUDA(ctx, cudaSetDevice(ctx->device));
+    B2N_TRY(ns_friends_alloc(ctx, ns));
+    StreamSwap swap_(ctx);
+    const int n = d.n, N = d.N;
+    const size_t nn = (size_t)n * n;
+    NsScalars h;                                 // round index: the bootstrap streams of this update
+    B2N_CUDA(ctx, b2n_copy_sync(ctx, &h, d.sc, sizeof(h), cudaMemcpyDeviceToHost));
+    if (!ns->fr_ready) {                         // no previous metric: the identity, RadFriends(ndim)'s (bounding.py:749-762)
+        std::vector<double> eye(nn, 0.0);
+        for (int i = 0; i < n; i++) eye[(size_t)i * n + i] = 1.0;
+        B2N_CUDA(ctx, b2n_copy_sync(ctx, ns->fr_am, eye.data(), nn * 8, cudaMemcpyHostToDevice));
+    }
+    const int mode = ctx->ptr_mode;
+    ctx->ptr_mode = B2N_PTR_DEVICE;              // the live set and the outputs are device arrays of this run
+    double lv = 0.0, r = 0.0;
+    int32_t ncl = 1;
+    // am_prev = the run's current am, overwritten in place by the new one (read by the first kernel of the update,
+    // written by its last copy, in stream order)
+    const int st = b2n_friends_update(ctx, d.live_u, N, n, kind, use_clustering, ns->fr_am, nboot, d.seed,
+                                      B2N_NS_FRIENDS_BOOT_CHAIN + ((unsigned long long)h.round << 8), ns->fr_cov, ns->fr_am,
+                                      ns->fr_axes, ns->fr_axinv, &lv, &r, &ncl);
+    ctx->ptr_mode = mode;
+    if (st != B2N_OK) return st;
+    if (enlarge != 1.0) {
+        // sampler.py:506-508: scale_to_logvol(logvol + ln enlarge), with the host class's arithmetic
+        // (f = exp(((L + ln e) - L) / n), not e^(1/n): (L + x) - L != x) so that both routes are bit-identical
+        const double T = lv + log(enlarge);
+        const double f = exp((T - lv) / (double)n);
+        B2N_TRY(b2n_friends_rescale_dev(ctx, n, ns->fr_cov, ns->fr_am, ns->fr_axes, ns->fr_axinv, f));
+        lv = T;
+    }
+    ns->fr_kind = kind;
+    ns->fr_logvol = lv;
+    ns->fr_radius = r;
+    ns->fr_ncl = ncl;
+    B2N_TRY(ns_friends_adopt(ctx, ns));
+    B2N_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (logvol) *logvol = lv;
+    if (radius) *radius = r;
+    if (nclusters) *nclusters = ncl;
+    return B2N_OK;
+}
+
+int b2n_ns_set_friends(b2n_ctx* ctx, int32_t kind, const double* cov, const double* am, const double* axes,
+                       const double* axes_inv, double logvol) {
+    if (!ctx || !ctx->ns || !ctx->ns->active || (kind != 0 && kind != 1) || !cov || !am || !axes || !axes_inv)
+        return B2N_ERR_ARG;
+    b2n_ns* ns = ctx->ns;
+    if (ns->d.nc != ns->d.n) return b2n_fail(ctx, B2N_ERR_ARG, "the friends bounds need ncdim == ndim");
+    B2N_CUDA(ctx, cudaSetDevice(ctx->device));
+    B2N_TRY(ns_friends_alloc(ctx, ns));
+    const size_t nn = (size_t)ns->d.n * ns->d.n * 8;
+    B2N_CUDA(ctx, cudaStreamSynchronize(ctx->stream));          // (enqueued rounds may still read the previous bound)
+    B2N_CUDA(ctx, b2n_copy_sync(ctx, ns->fr_cov, cov, nn, cudaMemcpyHostToDevice));
+    B2N_CUDA(ctx, b2n_copy_sync(ctx, ns->fr_am, am, nn, cudaMemcpyHostToDevice));
+    B2N_CUDA(ctx, b2n_copy_sync(ctx, ns->fr_axes, axes, nn, cudaMemcpyHostToDevice));
+    B2N_CUDA(ctx, b2n_copy_sync(ctx, ns->fr_axinv, axes_inv, nn, cudaMemcpyHostToDevice));
+    ns->fr_kind = kind;
+    ns->fr_logvol = logvol;
+    ns->fr_radius = NAN;                         // not known for an adopted bound
+    ns->fr_ncl = 0;
+    B2N_TRY(ns_friends_adopt(ctx, ns));
+    B2N_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return B2N_OK;
+}
+
+int b2n_ns_get_friends(b2n_ctx* ctx, double* cov, double* am, double* axes, double* axes_inv, double* logvol,
+                       double* radius, int32_t* nclusters) {
+    if (!ctx || !ctx->ns || !ctx->ns->active) return B2N_ERR_ARG;
+    b2n_ns* ns = ctx->ns;
+    if (!ns->fr_ready) return b2n_fail(ctx, B2N_ERR_ARG, "b2n_ns_get_friends: the run holds no friends bound");
+    B2N_CUDA(ctx, cudaSetDevice(ctx->device));
+    B2N_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    const size_t nn = (size_t)ns->d.n * ns->d.n * 8;
+    if (cov) B2N_CUDA(ctx, b2n_copy_sync(ctx, cov, ns->fr_cov, nn, cudaMemcpyDeviceToHost));
+    if (am) B2N_CUDA(ctx, b2n_copy_sync(ctx, am, ns->fr_am, nn, cudaMemcpyDeviceToHost));
+    if (axes) B2N_CUDA(ctx, b2n_copy_sync(ctx, axes, ns->fr_axes, nn, cudaMemcpyDeviceToHost));
+    if (axes_inv) B2N_CUDA(ctx, b2n_copy_sync(ctx, axes_inv, ns->fr_axinv, nn, cudaMemcpyDeviceToHost));
+    if (logvol) *logvol = ns->fr_logvol;
+    if (radius) *radius = ns->fr_radius;
+    if (nclusters) *nclusters = ns->fr_ncl;
     return B2N_OK;
 }
 

@@ -358,13 +358,26 @@ class NestedSampler:
         c = self.ctx if self.ctx is not None else m.ctx
         c.resident_key = m.version                     # these very ellipsoids ARE the resident bound
 
+    def _pull_device_friends(self, ctrs):
+        """Host RadFriends / SupFriends object <- the bound the device rounds hold; its centres are `ctrs` (the live
+        set the device bound was used with).  The ctx's resident axes stay anonymous: no host object claims them."""
+        from . import ops
+        o = ops.ns_get_friends(self.ndim, ctx=self.ctx)
+        b = self.bound
+        b.cov, b.am, b.axes, b.axes_inv, b.logvol = o['cov'], o['am'], o['axes'], o['axes_inv'], float(o['logvol'])
+        if o['nclusters'] > 0:                         # (an adopted bound reports none: the object's own values stand)
+            b.radius, b.nclusters = o['radius'], o['nclusters']
+        b.ctrs = ctrs
+        b.version = next(B._version)
+
     def _device_rounds(self, logz, logvol, loglstar, dlogz, maxiter, maxcall, batch, checkpoint_file=None,
                        checkpoint_every=0.0, snap=None, on_checkpoint=None, keep_samples=True, logl_max=None):
         """Run (or continue) with ``b2n_ns_run`` (include/b200nest.h): K-worst replacement rounds paced on the
         device -- first with prior draws (the phase before the first bound, sampler.py:407-409), then with the
         inner sampler against the resident bound.  The host only reacts to the device's flags: (re)build the bound
         (update_bound, sampler.py:493-510 -- on the device when ``_device_bound_ok``), grow the dead buffer, and
-        collect the dead points at the end."""
+        collect the dead points at the end.  With a RadFriends / SupFriends bound every update runs on the device
+        (``b2n_ns_update_friends``, bootstrap included) and a bound built beforehand is adopted as it is."""
         from . import ops
         import time
         n, N = self.ndim, self.nlive
@@ -390,6 +403,9 @@ class NestedSampler:
             it0_orig = snap['it0']
             it0 = it0_orig + len(prev[2])
         no_bound = self.bound_next is None
+        friends = isinstance(self.bound_next, B._B200Friends)
+        if friends and self.bound_bootstrap > 255:
+            raise ValueError("loop='device' with the friends bounds: bootstrap <= 255 (one chain id per realisation)")
         multi = not isinstance(self.bound_next, B.B200Ellipsoid)
         ops.ns_create(self.model.model_id(self.ctx), N, n, K, kind, steps, self.seed, chain0=chain_base,
                       ncdim=self.ncdim, strict_contains=multi,
@@ -410,7 +426,11 @@ class NestedSampler:
                 rounds0 = snap['rounds']
                 ops.ns_set_counters(snap['rounds'], snap['ncall_last_update'], snap['doubling'], ctx=self.ctx)
             if not self.unit_cube_sampling:
-                self._ensure_resident()
+                if friends:                           # resume / dynamic batch: the bound built so far, centred on the live set
+                    b = self.bound
+                    ops.ns_set_friends(b.kind, b.cov, b.am, b.axes, b.axes_inv, b.logvol, ctx=self.ctx)
+                else:
+                    self._ensure_resident()
             cap, last_forced = 64 * N, -1
             ncall_start, rounds = self.ncall, rounds0
             t_ckpt, n_ckpt, saved_it = time.perf_counter(), 0, 0
@@ -425,7 +445,10 @@ class NestedSampler:
                 saved_it = st['it']
                 if dev_nells:
                     self._pull_device_bound(dev_nells)
-                self._dev_snap = dict(dead=prev, live=ops.ns_get_live(N, n, ctx=self.ctx), logvol=st['logvol'],
+                live = ops.ns_get_live(N, n, ctx=self.ctx)
+                if friends:
+                    self._pull_device_friends(live[0])
+                self._dev_snap = dict(dead=prev, live=live, logvol=st['logvol'],
                                       logz=st['logz'], loglstar=st['loglstar'], ncall=st['ncall'], scale=st['scale'],
                                       rounds=st['rounds'], ncall_last_update=st['ncall_last_update'],
                                       doubling=st['doubling'], chain_base=chain_base, batch=K, it0=it0_orig)
@@ -466,7 +489,11 @@ class NestedSampler:
                         self.bound = self.bound_next
                         self.internal_sampler = self.internal_sampler_next
                         ncall_start, rounds0 = self.ncall, rounds      # calls per round change with the sampler
-                    if self._device_bound_ok():
+                    if friends:
+                        lv, _, _ = ops.ns_update_friends(self.bound.kind, self.bound_enlarge, self.bound_bootstrap,
+                                                         use_clustering=True, ctx=self.ctx)
+                        nells = 1
+                    elif self._device_bound_ok():
                         dev_nells, lv, warn = ops.ns_update_bound(multi, self.bound_enlarge, ctx=self.ctx)
                         nells = dev_nells
                     else:
@@ -492,6 +519,8 @@ class NestedSampler:
                 if dev_nells:
                     self._pull_device_bound(dev_nells)
             self.live_u, self.live_v, self.live_logl = ops.ns_get_live(N, n, ctx=self.ctx)
+            if friends and not self.unit_cube_sampling:
+                self._pull_device_friends(self.live_u)
             new = ops.ns_get_dead(saved_it, st['it'] - saved_it, n, ctx=self.ctx, positions=keep_samples)
             out = tuple(np.concatenate([a, b]) for a, b in zip(prev, new))
             self.chain_counter = chain_base + rounds * K

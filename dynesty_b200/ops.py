@@ -446,6 +446,47 @@ def ns_get_bound(nells, ncdim, ctx=None):
     return o
 
 
+_FRIENDS_KIND = {'balls': 0, 'cubes': 1}
+
+
+def ns_update_friends(kind, enlarge=1.0, nboot=0, use_clustering=True, ctx=None):
+    """RadFriends / SupFriends update on the device (b2n_ns_update_friends): fit to the run's live points in HBM under
+    the run's previous metric, enlarge, make it the run's bound.  kind: 'balls' | 'cubes'.
+    Returns (logvol, radius, nclusters)."""
+    ctx = _ctx(ctx)
+    lv, rad, ncl = C.c_double(0.0), C.c_double(0.0), C.c_int32(0)
+    ctx.resident_key = None
+    ctx.check(ctx.lib.b2n_ns_update_friends(ctx.h, _FRIENDS_KIND[kind], float(enlarge), int(nboot), int(bool(use_clustering)),
+                                            C.addressof(lv), C.addressof(rad), C.addressof(ncl)))
+    _ns_bound_serial[0] += 1
+    ctx.resident_key = ('ns', ctx.serial, _ns_bound_serial[0])     # the run's common axes; no host object owns them
+    return lv.value, rad.value, ncl.value
+
+
+def ns_set_friends(kind, cov, am, axes, axes_inv, logvol, ctx=None):
+    """Adopt a RadFriends / SupFriends bound built on the host as the run's bound (centres: the run's live set)."""
+    ctx = _ctx(ctx)
+    cov, am, axes, axes_inv = f64(cov), f64(am), f64(axes), f64(axes_inv)
+    ctx.resident_key = None
+    ctx.check(ctx.lib.b2n_ns_set_friends(ctx.h, _FRIENDS_KIND[kind], ptr(cov), ptr(am), ptr(axes), ptr(axes_inv),
+                                         float(logvol)))
+    _ns_bound_serial[0] += 1
+    ctx.resident_key = ('ns', ctx.serial, _ns_bound_serial[0])
+
+
+def ns_get_friends(ndim, ctx=None):
+    """The friends bound the run holds: dict(cov, am, axes, axes_inv, logvol, radius, nclusters) (an adopted bound:
+    radius nan, nclusters 0)."""
+    ctx = _ctx(ctx)
+    n = int(ndim)
+    o = dict(cov=np.empty((n, n)), am=np.empty((n, n)), axes=np.empty((n, n)), axes_inv=np.empty((n, n)))
+    lv, rad, ncl = C.c_double(0.0), C.c_double(0.0), C.c_int32(0)
+    ctx.check(ctx.lib.b2n_ns_get_friends(ctx.h, ptr(o['cov']), ptr(o['am']), ptr(o['axes']), ptr(o['axes_inv']),
+                                         C.addressof(lv), C.addressof(rad), C.addressof(ncl)))
+    o.update(logvol=lv.value, radius=rad.value, nclusters=ncl.value)
+    return o
+
+
 def ns_reserve_dead(capacity, ctx=None):
     ctx = _ctx(ctx)
     ctx.check(ctx.lib.b2n_ns_reserve_dead(ctx.h, int(capacity)))

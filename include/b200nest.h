@@ -421,6 +421,32 @@ int b2n_ns_update_bound(b2n_ctx* ctx, int32_t multi, double enlarge, int32_t* ne
 /* the bound b2n_ns_update_bound built last (host outputs sized for max_ells >= nells; each may be NULL) */
 int b2n_ns_get_bound(b2n_ctx* ctx, int32_t max_ells, double* ctrs, double* covs, double* ams, double* axes,
                      double* axlens, double* logvols);
+/* ---- friends mode: RadFriends / SupFriends bounds (kind 0 balls, 1 cubes; ncdim == ndim) in the rounds.
+ * b2n_ns_create starts every run in ellipsoid mode; the first of the two entry points below that installs a bound
+ * switches the run to friends mode for the rest of its life (b2n_ns_update_bound is then refused).  In this mode the
+ * bound is one ball / cube of common shape (cov, am, axes, axes_inv) around EVERY live point as the live set stands
+ * (the reference re-points bound.ctrs = live_u before every proposal, sampler.py:479-482).  A round's chains all use
+ * the common axes (get_random_axes); there is no contains test of the start points: a start is a live point, hence a
+ * centre (distance 0), so the forced update of sampler.py:485-489 cannot fire.  With sampler 3 every chain draws with
+ * RadFriends.sample / SupFriends.sample (bounding.py:797-831 / 1065-1100) around the run's live set, accepted with
+ * probability 1/q; the round's commit keeps the transformed centres of the replaced rows current.
+ *
+ * b2n_ns_update_friends = Sampler.update_bound (sampler.py:493-510) without leaving the device: b2n_friends_update on
+ * the run's live set in HBM with am_prev = the run's current am (the identity before the first bound), then
+ * scale_to_logvol(logvol + ln enlarge) (the host class's arithmetic: both routes give the same bits).  Bootstrap
+ * realisation b (nboot <= 255, else B2N_ERR_ARG) of an update made at round r draws its resample from the B2N chain
+ * (seed, 0x6000000000000000 + (r << 8) + b).  logvol / radius / nclusters: host outputs, may be NULL.  Follow with
+ * b2n_ns_bound_updated.  Synchronises.
+ * b2n_ns_set_friends adopts a bound built elsewhere (host arrays, n x n each) as the run's bound, its centres being the
+ * run's live set: a restored run, a dynamic-sampler batch, a host-route update.
+ * b2n_ns_get_friends returns the bound the run holds (host outputs, each may be NULL; an adopted bound reports radius
+ * NaN and nclusters 0). */
+int b2n_ns_update_friends(b2n_ctx* ctx, int32_t kind, double enlarge, int32_t nboot, int32_t use_clustering,
+                          double* logvol, double* radius, int32_t* nclusters);
+int b2n_ns_set_friends(b2n_ctx* ctx, int32_t kind, const double* cov, const double* am, const double* axes,
+                       const double* axes_inv, double logvol);
+int b2n_ns_get_friends(b2n_ctx* ctx, double* cov, double* am, double* axes, double* axes_inv, double* logvol,
+                       double* radius, int32_t* nclusters);
 /* grow the dead-point buffer to `capacity` rows (keeps the rows written so far); clears need_bound == 3 */
 int b2n_ns_reserve_dead(b2n_ctx* ctx, int64_t capacity);
 /* host outputs (each may be NULL) */
